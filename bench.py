@@ -8,6 +8,7 @@ of the full-resolution scan, vertex append, per-voxel dilation / Delaunay / pull
   python bench.py --gpus 1 --steps K --warmup W               our CUDA path (N>1: launched under torchrun)
   python bench.py --impl reference --gpus 1 --steps K ...     the reference algorithm on the host cores (oracle port)
   python bench.py --config C1|C2|C3|C4|C5|C5s1                the other BASELINE.json configurations (default: the 100k metric config)
+  python bench.py ... --dump-outputs DIR                      also write what the timed path returned after its last step as DIR/*.npy
 
 Prints ONE JSON line (rank 0).  `value` = scans/s with the scans already resident in HBM (device-event time, L2
 flushed between scans); `e2e` = scans/s through the C ABI with pinned HOST buffers (H2D of both clouds and D2H of the
@@ -201,8 +202,9 @@ def cpu_thread_sets():
     return [("all", min(16, n), min(64, n)), ("ref4", min(4, n), min(64, n))]
 
 
-def run_cpu(wl, scans, n_warm, n_timed, t_loc, t_mesh):
-    """The reference algorithm on the host cores (oracle port): returns per-scan (t_loc, t_mesh) seconds."""
+def run_cpu(wl, scans, n_warm, n_timed, t_loc, t_mesh, dump_dir=None):
+    """The reference algorithm on the host cores (oracle port): returns per-scan (t_loc, t_mesh) seconds.  dump_dir: write the
+    state and mesh after the last scan there (dump_outputs)."""
     from oracle_api import OracleLio, OracleMesh
     cfg = wl["lio"]
     lio = OracleLio(cfg, sum_mode=1, omp_threads=t_loc, solve_mode=1, plane_var_mode=1)   # the reference's literal formulation: serial double sums, two 18x18 inverses, per-point plane covariance loop
@@ -214,7 +216,7 @@ def run_cpu(wl, scans, n_warm, n_timed, t_loc, t_mesh):
         sc = scans[k]
         t0 = time.perf_counter()
         lio.predict(sc["dt"])
-        lio.lio_state_estimation(sc["body_ds"])
+        iters = lio.lio_state_estimation(sc["body_ds"])
         lio.map_incremental_grow(sc["body_ds"])
         t1 = time.perf_counter()
         world = lio.transform_full(sc["body_full"])                 # transformLidar of the full scan
@@ -222,6 +224,10 @@ def run_cpu(wl, scans, n_warm, n_timed, t_loc, t_mesh):
         t2 = time.perf_counter()
         if k > n_warm:
             times.append((t1 - t0, t2 - t1))
+    if dump_dir:
+        verts, tris, flags = mesh.snapshot()
+        dump_outputs(dump_dir, {"state": lio.get_state(), "iterations": [iters]},
+                     {"mesh_vertices": verts, "mesh_triangles": tris, "mesh_triangle_flags": flags})
     return np.array(times)
 
 
@@ -294,6 +300,26 @@ def algorithmic_bytes(kernel, info):
     if kernel == "k_transform_full":
         return 24.0 * info["n_full"]
     return None
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, fixed, rows):
+    """--dump-outputs: every array as out_dir/<name>.npy, float32 kept, everything else as float64 (integers up to 2^53 exactly).
+    `rows` are per-row tables (vertices, facets, ...); if the whole dump would exceed DUMP_BYTES, each of them keeps the same
+    fraction of its rows, chosen by a fixed seed and kept in order, so that two runs with the same arguments write the same files
+    and tables of equal length keep the same rows."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {**fixed, **rows}
+    arrays = {n: np.asarray(a, dtype=np.float32 if np.asarray(a).dtype == np.float32 else np.float64) for n, a in arrays.items()}
+    fixed_bytes = sum(arrays[n].nbytes for n in fixed)
+    row_bytes = sum(arrays[n].nbytes for n in rows)
+    frac = min(1.0, (DUMP_BYTES - fixed_bytes) / row_bytes) if row_bytes else 1.0
+    for name, a in arrays.items():
+        if name in rows and frac < 1.0:
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], int(a.shape[0] * frac), replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def pin(a):
@@ -434,7 +460,7 @@ def run_gpu(args, rank, world):
     MW = wl["map_warm"]
     n_prof = min(K, 10)
     n_stage = min(K, 10)
-    K_raw = 0 if args.no_raw_leg else min(K, 20)
+    K_raw = 0 if args.no_raw_leg else K
     n_scans = 1 + MW + W + 2 * K + K_raw + n_stage + n_prof + 1 + 6 + K + K_raw    # the last K + K_raw: a second pass of a host-buffer leg (below)
     scans = get_stream(wl, n_scans, seed=rank if args.independent_streams else 0)
     lib = api.load_library()
@@ -515,10 +541,14 @@ def run_gpu(args, rank, world):
     waits = api.host_wait_ms(lio, mesh)
     host_enqueue_ms = (enq_wall_ms - sum(waits)) / K     # host WORK to queue one scan; the waits are back-pressure from the 2-deep staging slots
     total_ms = api.pipeline_mark_end(lio, mesh)
-    lio.wait()
+    state, iters = lio.wait()
     mesh.wait()
     barrier()
     launches = api.launch_count(lib) - launches0
+    if args.dump_outputs and rank == 0:      # what a caller of the timed path holds after its last step
+        verts, tris, flags = mesh.snapshot()
+        dump_outputs(args.dump_outputs, {"state": state, "iterations": [iters]},
+                     {"mesh_vertices": verts, "mesh_triangles": tris, "mesh_triangle_flags": flags})
     # the flush alone, to report how much of the timed region it is
     api.pipeline_mark_begin(lio)
     for _ in range(K):
@@ -764,10 +794,11 @@ def run_reference(args, rank, world):
     K = args.steps if args.steps is not None else wl["steps"]
     W = max(args.warmup, 3)
     MW = wl["map_warm"]
-    K_eff = min(K, 40 if args.config in ("C100k", "C1", "C2") else 8)      # bounded so that the run ends within a few minutes
+    # without --steps: bounded so that the run ends within a few minutes
+    K_eff = args.steps if args.steps is not None else min(K, 40 if args.config in ("C100k", "C1", "C2") else 8)
     scans = get_stream(wl, 1 + min(MW, 4) + W + K_eff + 1)
     label, tl, tm = cpu_thread_sets()[0]
-    tt = run_cpu(wl, scans, min(MW, 4) + W, K_eff, tl, tm)
+    tt = run_cpu(wl, scans, min(MW, 4) + W, K_eff, tl, tm, dump_dir=args.dump_outputs)
     sm = cpu_summary(tt)
     v = sm["pipelined_scans_s"]
     out = {"impl": "reference", "metric": METRIC if args.config == "C100k" else f"scans/sec loc+mesh ({args.config})", "value": v, "unit": "scans/s", "n_gpus": world,
@@ -796,6 +827,9 @@ def main():
     ap.add_argument("--no-parity-gate", action="store_true", help="experiments only: skip the GPU-vs-oracle check that precedes the timed regions")
     ap.add_argument("--streams", type=int, default=None, help="N=1: also measure this many independent streams interleaved on the one GPU (reported as `multi_stream`; 1 = skip)")
     ap.add_argument("--no-sharded-extra", action="store_true", help="N>1, replicas mode: skip the additional sharded single-stream measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path returned after its last step (state, iteration count, mesh vertices / facets / "
+                         "orientation flags) as DIR/<name>.npy, at most 64 MB in all (a seeded sample of the mesh rows beyond that)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))

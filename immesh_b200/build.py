@@ -13,7 +13,6 @@ CSRC = os.path.join(_HERE, "csrc")
 LIB = os.path.join(_HERE, "libimmesh_b200.so")
 EMU = os.path.join(_ROOT, "tests", "emu", "libimmesh_emu.so")
 ORACLE = os.path.join(_ROOT, "oracle", "liborc.so")
-REF_IKD = os.path.join(_ROOT, "oracle", "_ref", "libref_ikd.so")
 GXX = "/usr/bin/g++"
 
 NVCC_FLAGS = [
@@ -64,19 +63,10 @@ def build_emu(force=False):
     return EMU
 
 
-def build_ref():
-    """oracle/_ref: the reference's own ikd-Tree compiled unmodified from /root/reference (only in the authoring container;
-    the GPU box uses the prebuilt file that travels with the snapshot)."""
-    if os.path.isdir("/root/reference/include/ikd-Tree"):
-        subprocess.check_call(["make", "-s", "-C", os.path.join(_ROOT, "oracle"), "-f", "Makefile.ref"])
-    return REF_IKD
-
-
 def build_all(force=False):
     build_cuda(force)
     build_oracle(force)
     build_emu(force)
-    build_ref()
 
 
 if __name__ == "__main__":

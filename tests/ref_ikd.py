@@ -1,7 +1,7 @@
 """ctypes wrapper over oracle/_ref/libref_ikd.so -- the REFERENCE's own ikd-Tree (include/ikd-Tree/ikd_Tree.{h,cpp}) compiled
-unmodified by oracle/Makefile.ref.  Test infrastructure only.  The library is (re)built when /root/reference is present (this
-container); on the GPU box only the prebuilt file is used.  `available()` is False when neither exists (tests then skip and
-the committed fixtures under tests/golden/ carry the pin)."""
+unmodified from an ImMesh checkout by oracle/Makefile.ref.  tools/make_golden.py drives it to produce the fixtures under
+tests/golden/; the tests compare against those fixtures and need neither the library nor the checkout.  `same_knn` is the
+kNN comparison they use."""
 import ctypes as C
 import os
 import subprocess
@@ -13,24 +13,17 @@ _SO = os.path.join(_ROOT, "oracle", "_ref", "libref_ikd.so")
 _lib = None
 
 
-def build():
-    if os.path.isdir("/root/reference/include/ikd-Tree"):
-        subprocess.check_call(["make", "-s", "-C", os.path.join(_ROOT, "oracle"), "-f", "Makefile.ref"])
-    return os.path.exists(_SO)
-
-
-def available():
-    try:
-        return build()
-    except Exception:
-        return os.path.exists(_SO)
+def build(ref_dir):
+    """Compile oracle/_ref/libref_ikd.so from the ImMesh checkout at ref_dir."""
+    subprocess.check_call(["make", "-s", "-C", os.path.join(_ROOT, "oracle"), "-f", "Makefile.ref", f"REF={os.path.abspath(ref_dir)}"])
+    return _SO
 
 
 def lib():
     global _lib
     if _lib is None:
-        if not available():
-            raise RuntimeError("oracle/_ref/libref_ikd.so is not built")
+        if not os.path.exists(_SO):
+            raise RuntimeError("oracle/_ref/libref_ikd.so is not built (ref_ikd.build)")
         L = C.CDLL(_SO)
         L.ref_ikd_create.restype = C.c_void_p
         L.ref_ikd_destroy.argtypes = [C.c_void_p]

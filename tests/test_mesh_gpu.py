@@ -55,20 +55,15 @@ def test_golden_reference_ikdtree_append_and_knn(cuda_lib):
 
 
 def test_knn_matches_reference_ikdtree_live(cuda_lib):
-    """CUDA kNN against the reference ikd-Tree library itself (oracle/_ref travels with the snapshot)."""
+    """CUDA kNN over the vertices of three meshed frames against the reference ikd-Tree built on the same vertices
+    (tests/golden/ikd_mesh_knn.npz, tools/make_golden.py)."""
     import ref_ikd
-    if not ref_ikd.available():
-        pytest.skip("oracle/_ref/libref_ikd.so not present")
+    gk = _golden("ikd_mesh_knn.npz")
     g, o, _ = run_mesh_parity(cuda_lib, "avia", 3, seed=9)
-    v = g.snapshot()[0]
-    t = ref_ikd.RefIkdTree()
-    t.add(v)
-    rng = np.random.default_rng(1)
-    q = (v[rng.integers(0, len(v), 4000)] + rng.normal(0, 0.2, (4000, 3))).astype(np.float32)
-    for k, md in ((20, np.inf), (1, 0.1), (20, 1.0)):
-        ig, dg = g.knn(q, k, md)
-        ir, dr, _ = t.knn(q, k, md)
-        assert ref_ikd.same_knn(ig.astype(np.int64), dg, ir, dr), (k, md)
+    assert g.counts()["n_vertices"] == int(gk["n_vertices"])
+    for c, (k, md) in enumerate(gk["cases"]):
+        ig, dg = g.knn(gk["queries"], int(k), float(md))
+        assert ref_ikd.same_knn(ig.astype(np.int64), dg, gk[f"idx{c}"].astype(np.int64), gk[f"d2{c}"]), (k, md)
 
 
 def test_empty_frame_and_restart(cuda_lib):

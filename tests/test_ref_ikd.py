@@ -1,20 +1,15 @@
-"""Pins the kNN / vertex-append rows of the oracle (SURVEY 8a a13-a15) to the REFERENCE's own ikd-Tree.
-
-* live: oracle vs oracle/_ref/libref_ikd.so (include/ikd-Tree/ikd_Tree.cpp compiled unmodified, oracle/Makefile.ref) --
-  skipped where the library is neither built nor buildable;
-* golden: oracle vs tests/golden/ikd_*.npz, generated from the same library by tools/make_golden.py (always runs).
-The CUDA path is checked against the same fixtures in tests/test_mesh_gpu.py."""
+"""Pins the kNN / vertex-append rows of the oracle (SURVEY 8a a13-a15) to the REFERENCE's own ikd-Tree: the oracle against
+tests/golden/ikd_*.npz, generated from include/ikd-Tree/ikd_Tree.cpp compiled unmodified (oracle/Makefile.ref) by
+tools/make_golden.py.  The CUDA path is checked against the same fixtures in tests/test_mesh_gpu.py."""
 import os
 
 import numpy as np
-import pytest
 
 import oracle_api as oa
 import ref_ikd
 from immesh_b200 import api, synth
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-needs_ref = pytest.mark.skipif(not ref_ikd.available(), reason="oracle/_ref/libref_ikd.so not built and /root/reference absent")
 
 
 def _oracle_with_frames(frames, pose_t, cfg):
@@ -43,33 +38,27 @@ def test_golden_knn_matches_oracle():
         assert ref_ikd.same_knn(idx.astype(np.int64), d2, g[f"idx{c}"].astype(np.int64), g[f"d2{c}"]), (k, md)
 
 
-@needs_ref
 def test_oracle_knn_matches_reference_ikdtree_incremental():
+    """The tree grown frame by frame with the oracle's new vertices, queried after every frame."""
+    g = np.load(os.path.join(GOLD, "ikd_incremental.npz"))
     sensor, scans = synth.make_stream("avia", 4, seed=11, n_points=12000)
     frames = [(s["body_full"].astype(np.float64) @ s["R_true"].T + s["t_true"]).astype(np.float32) for s in scans]
-    o, t, n_prev = oa.OracleMesh(api.MeshConfig()), ref_ikd.RefIkdTree(), 0
-    rng = np.random.default_rng(5)
+    o = oa.OracleMesh(api.MeshConfig())
     for k, f in enumerate(frames):
         o.push_frame(f, scans[k]["t_true"], k)
         v, _, _ = o.snapshot()
-        t.add(v[n_prev:])            # Add_Point per accepted vertex, as pointcloud_rgbd.cpp:540 (tree re-balances itself)
-        n_prev = len(v)
-        q = (v[rng.integers(0, len(v), 1500)] + rng.normal(0, 0.15, (1500, 3))).astype(np.float32)
-        for kk, md in ((20, float("inf")), (1, 0.1), (20, 1.0), (5, 0.3)):
-            io, do = o.knn(q, kk, md)
-            ir, dr, _ = t.knn(q, kk, md)
-            assert ref_ikd.same_knn(io.astype(np.int64), do, ir, dr), (k, kk, md)
+        assert len(v) == int(g[f"n_vertices{k}"]), k       # the vertex set the reference tree was grown with
+        for c, (kk, md) in enumerate(g["cases"]):
+            io, do = o.knn(g[f"queries{k}"], int(kk), float(md))
+            assert ref_ikd.same_knn(io.astype(np.int64), do, g[f"idx{k}_{c}"].astype(np.int64), g[f"d2{k}_{c}"]), (k, kk, md)
 
 
-@needs_ref
 def test_oracle_append_matches_reference_ikdtree_driven_loop():
-    import sys
-    sys.path.insert(0, os.path.join(os.path.dirname(GOLD), "..", "tools"))
-    from make_golden import append_with_tree
+    """The append loop with the reference tree answering its 1-NN queries (tools/make_golden.py append_with_tree)."""
+    ref = np.load(os.path.join(GOLD, "ikd_loop.npz"))["verts"]
     cfg = api.MeshConfig()
     sensor, scans = synth.make_stream("avia", 3, seed=4, n_points=4000)
     frames = [(s["body_full"].astype(np.float64) @ s["R_true"].T + s["t_true"]).astype(np.float32) for s in scans]
-    ref = append_with_tree(frames, cfg.points_minimum_scale, cfg.number_of_pts_append_to_map)
     o = _oracle_with_frames(frames, [s["t_true"] for s in scans], cfg)
     v, _, _ = o.snapshot()
     assert v.shape == ref.shape and np.array_equal(v, ref)
